@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the PathTrace hot path (BASELINE.json: "Mrays/s and ms/frame @1080p 4spp 6-bounce Bistro").
 
   python bench.py --gpus N --steps K --warmup W            product arm (CUDA wavefront through the C ABI)
+      [--dump-outputs DIR]                                 ... and write the frame the last timed step produced to DIR/accumulated.npy
   python bench.py --impl reference --gpus N ...            reference arm: the reference's algorithm for this path on the host cores
                                                            (RTXPT itself has no CPU implementation and cannot run here — HLSL/DXR, Windows
                                                            only, SURVEY.md F1-F3 — so this arm times the CPU restatement in oracle/)
@@ -10,7 +11,8 @@ Workload (configs[1] of BASELINE.json, fits one GPU): 1920x1080, 4 sub-samples p
 NEE with 5 candidates + 1 shadow ray per vertex, Russian roulette, firefly filter on, environment map on, on the ~2.8 M triangle procedural
 "city block" stand-in for Bistro exterior (the real Bistro assets are git-LFS stubs in the reference tree: SURVEY.md F7).
 A step is one frame: 4 sub-samples path traced and folded into the accumulation buffer.  A ray is one traversal query (scatter or shadow).
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  The scene is generated from fixed seeds and frame i uses sample indices 4i..4i+3, so the same arguments give the
+same inputs on every run; the benchmark writes nothing into the source tree (the tree may be read-only).
 """
 import argparse
 import ctypes as C
@@ -24,6 +26,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True          # no __pycache__ in the tree
 
 import numpy as np
 
@@ -186,8 +189,7 @@ def physical_cores():
 
 def run_cpu(scene, consts, steps, warmup):
     """Times the oracle (CPU restatement of the reference path, OpenMP over all host cores) on the bounded sample; returns Mrays/s etc."""
-    import oracle_lib as ol
-    ol.build()
+    import oracle_lib as ol             # the library build() made; not rebuilt here
     t0 = time.time(); o = ol.Oracle(scene); bvh_s = ol.lib().oracle_bvh_build_seconds(o.h)
     o.set_constants(consts); setup_s = time.time() - t0
     rect = cpu_sample_rect()
@@ -210,12 +212,19 @@ def run_cpu(scene, consts, steps, warmup):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=int, default=30, help="timed frames of the headline and end-to-end measurements (and of --impl reference); the CPU baseline "
+                                                           "(3 steps) and the realtime child (scripts/bench_realtime.py, 10 frames) keep their own counts")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-realtime", action="store_true", help="skip the realtime-mode (stable planes) timing that runs in a child process after the headline measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the accumulated RGBA float32 frame the last timed step left (what a caller reads back) "
+                                                           "to DIR/accumulated.npy, so that two builds can be compared on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA arm (--impl b200)")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     n_gpus = args.gpus
 
@@ -299,6 +308,11 @@ def main():
     else:
         rays_per_frame = float(rays_per_frame_local)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        # after the clock sampler (the GPU idles during the file write) and before the e2e leg (which keeps accumulating into the same buffer); rank 0 holds
+        # the whole frame (N > 1: after the all-gather of the last step); 1920 x 1080 x 4 float32 = 33 MB
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "accumulated.npy"), ctx.readback_accumulated())
     ms_per_step = ms_total / args.steps
     value = rays_per_frame / (ms_per_step * 1e-3) / 1e6
 
@@ -383,7 +397,7 @@ def main():
     if rank == 0 and world == 1 and not args.no_realtime:
         # realtime mode (row a17) timed in a child process on the same workload: a fault there cannot take the headline line with it
         try:
-            r = subprocess.run([sys.executable, os.path.join(os.path.dirname(os.path.abspath(__file__)), "scripts", "bench_realtime.py")], capture_output=True, text=True, timeout=300)
+            r = subprocess.run([sys.executable, "-B", os.path.join(os.path.dirname(os.path.abspath(__file__)), "scripts", "bench_realtime.py")], capture_output=True, text=True, timeout=300)
             # the child prints its line before tearing the context down, so a fault in its last (never-before-run) stage still leaves the measurements
             realtime = json.loads(r.stdout.strip().splitlines()[-1]) if r.stdout.strip() else {"error": "exit %d: %s" % (r.returncode, r.stderr.strip()[-300:])}
             if r.returncode != 0: realtime["child_exit"] = r.returncode

@@ -1,7 +1,7 @@
 """CPU: the oracle's integer / packing primitives against the reference's own known answers.
   - tests/golden/rng_golden.json: produced from the UNMODIFIED NoiseAndSequences.hlsli C++ half (tests/golden/make_rng_golden.py)
   - fp16 known answers of External/Donut/tests/src/engine/test_float.cpp:74-90 (round-to-nearest-even f32->f16)
-  - when /root/reference is present (build container) the golden file is regenerated and must be identical (pins the fixture itself)"""
+  - where build() compiled oracle/_ref/ from the reference sources, the golden file is regenerated and must be identical (pins the fixture itself)"""
 import json
 import os
 import subprocess
@@ -34,12 +34,17 @@ def test_sobol_against_reference_header(oracle):
         assert L.oracle_sobol(index, dim) == v
 
 
-def test_golden_file_matches_reference_tree():
-    ref = "/root/reference/Rtxpt/Shaders/PathTracer/Utils/NoiseAndSequences.hlsli"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not present (GPU box)")
+def _ref_binary(name):
+    """oracle/_ref/<name>, compiled by build() (make -C oracle ref) where the reference sources are present; the test skips where it was never built."""
     subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "ref"], check=True)
-    out = subprocess.run([os.path.join(ROOT, "oracle", "_ref", "ref_kat")], check=True, capture_output=True, text=True).stdout
+    exe = os.path.join(ROOT, "oracle", "_ref", name)
+    if not os.path.exists(exe):
+        pytest.skip("oracle/_ref/%s not built (build() compiles it only where the reference sources are present)" % name)
+    return exe
+
+
+def test_golden_file_matches_reference_tree():
+    out = subprocess.run([_ref_binary("ref_kat")], check=True, capture_output=True, text=True).stdout
     fresh = json.loads(out); g = golden()
     for k in ("hash32", "hash32_combine", "sobol"):
         assert fresh[k] == g[k]
@@ -146,9 +151,7 @@ def test_material_building_blocks_equal_the_reference_headers_bit_for_bit(oracle
 
 
 def test_bsdf_golden_file_matches_reference_tree():
-    if not os.path.exists("/root/reference/Rtxpt/Shaders/PathTracer/Rendering/Materials/BxDF.hlsli"):
-        pytest.skip("reference tree not present (GPU box)")
-    subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "ref"], check=True)
+    _ref_binary("ref_kat_bsdf")
     import importlib.util
     spec = importlib.util.spec_from_file_location("make_bsdf_golden", os.path.join(HERE, "golden", "make_bsdf_golden.py")); m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m)
     rec, out, u, fout = m.generate(); g = bsdf_golden()

@@ -1,12 +1,13 @@
 """RTXPT .scene.json loading (rtxpt_b200_load_scene_json): models instanced through the graph with translation / rotation / euler / scaling,
 lights, cameras, environment light and settings — against the same scene assembled with the numpy table builder.  CPU only."""
+import gzip
 import json
 import os
 import numpy as np
 import pytest
 import gltf_export
 
-REF_ASSETS = "/root/reference/Assets"
+ASSETS_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_assets.json.gz")
 
 
 def _quat_matrix(q):
@@ -102,13 +103,19 @@ def test_scene_json_errors(product, tmp_path):
         product.GltfScene(str(p))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_ASSETS), reason="reference assets not present")
-def test_reference_scene_files_parse_up_to_their_lfs_stubs(product):
-    """Every .scene.json the reference ships is read up to the point where its models (git-LFS pointer stubs in this checkout) would be parsed."""
-    import glob
-    files = sorted(glob.glob(os.path.join(REF_ASSETS, "*.scene.json")))
+def test_reference_scene_files_parse_up_to_their_lfs_stubs(product, tmp_path):
+    """Every .scene.json the reference ships is read up to the point where its models (git-LFS pointer stubs in the reference checkout) would be parsed.
+    The scene files and the stubs they name are laid out again under tmp_path from tests/golden/reference_assets.json.gz.  The expected messages there
+    (scene_errors) were recorded from this project's own loader on the reference's Assets tree, not from the reference: they pin the loader's current
+    wording as a regression check, and a deliberate rewording of a loader error means regenerating them (tests/golden/make_asset_golden.py)."""
+    with gzip.open(ASSETS_GOLDEN, "rt", encoding="utf-8") as f:
+        golden = json.load(f)
+    for name, text in list(golden["scenes"].items()) + list(golden["models"].items()):
+        p = tmp_path / name; p.parent.mkdir(parents=True, exist_ok=True); p.write_text(text, encoding="utf-8")
+    files = sorted(golden["scenes"])
     assert len(files) >= 8
     for f in files:
         with pytest.raises(product.RtxptError) as e:
-            product.GltfScene(f)
+            product.GltfScene(str(tmp_path / f))
         assert "JSON" in str(e.value) or "cannot open" in str(e.value), (f, str(e.value))          # the stub is not JSON / the file is absent; never a crash
+        assert str(e.value) == golden["scene_errors"][f].replace("{assets}", str(tmp_path)), (f, str(e.value))
